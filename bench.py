@@ -17,14 +17,15 @@ Printed JSON (one line, rank 0): the base contract keys plus
                 mean launch time measured with CUDA events inside real steps, against BOTH measured bf16 peaks of
                 MEASURED_PEAKS.json (burst and sustained); step-level fractions beside it
   parity        the step's own output checked in the run: the first CPU_SAMPLE_BATCH samples of the SAME inputs go
-                through the reference (baseline/_ref, fp32 on the host) and are compared with the GPU prediction
+                through the reference (oracle/_ref, fp32 on the host) and are compared with the GPU prediction
   cpu_baseline  the reference's own CPU path timed on that bounded sample (N=1 only)
   e2e           the same metric with HOST buffers: pinned-host -> device copy of the step's inputs and device ->
                 pinned-host copy of the full prediction inside the timed region (double-buffered on side streams)
   secondary     the other quantities BASELINE.json's metric names: RVQ Mcodes/s (configs[3], 1M frames, bit-exact
                 sample check, own roofline) and the conditional denoiser (configs[2], B=16) steps/s
-`--impl reference` times the reference arm: the UNMODIFIED reference (pip-installed into baseline/_ref, third-party
+`--impl reference` times the reference arm: the UNMODIFIED reference (pip-installed into oracle/_ref, third-party
 imports it does not need on this path stubbed) on the host cores, same metric/unit/config; rank 0 only.
+`--dump-outputs DIR` writes what the last timed step computed on rank 0 as DIR/<name>.npy (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -51,6 +52,7 @@ FF_INNER = 1365                      # int(512 * 4 * 2 / 3)
 CONV_FLOPS_PER_LAUNCH = 2.0 * BATCH * SEQ * FF_INNER * (3 * FF_INNER)   # algorithmic (unpadded) FLOPs
 WORKLOAD = "configs[1]: Model(dim=512, depth=12, heads=8) unconditional, bf16 operands, seq=1024, batch=32 per GPU"
 CPU_SAMPLE_BATCH = 4   # bounded sample of the 32-sample workload step for the in-run CPU legs
+DUMP_ROWS = 8192       # --dump-outputs keeps this many of the 32 x 1024 prediction rows (16 MiB of the 64 MiB)
 
 
 def build_config(world: int) -> dict:
@@ -128,7 +130,7 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------------------
-# the reference (baseline/_ref) on the host
+# the reference (oracle/_ref) on the host
 # ------------------------------------------------------------------------------------------------------
 def _host_threads() -> int:
     """CPU threads this process may really use: affinity mask, capped by the cgroup CPU quota (oversubscribing a
@@ -144,11 +146,12 @@ def _host_threads() -> int:
 
 
 def import_reference():
-    """The unmodified reference package from baseline/_ref (`pip install --no-deps --target baseline/_ref`, recorded
-    in DESIGN.md).  Third-party modules it imports at module scope but never touches on the denoiser path are
+    """The unmodified reference package from oracle/_ref (`pip install --no-deps --target oracle/_ref`, see
+    oracle/reference.py).  Third-party modules it imports at module scope but never touches on the denoiser path are
     stubbed (SURVEY Appendix A).  Returns the `naturalspeech2_pytorch.naturalspeech2_pytorch` module or None."""
-    ref_dir = ROOT / "baseline" / "_ref"
-    if not (ref_dir / "naturalspeech2_pytorch").exists():
+    from oracle import reference
+    ref_dir = reference.REF_DIR
+    if not reference.installed():
         return None
     import torch
 
@@ -189,7 +192,7 @@ def import_reference():
 
 
 class HostReference:
-    """The reference denoiser on the host cores: baseline/_ref when importable (kind 'reference'), else the
+    """The reference denoiser on the host cores: oracle/_ref when importable (kind 'reference'), else the
     torch port of the oracle (kind 'port').  Same fp32 weights as the GPU model (state_dict keys are identical)."""
 
     def __init__(self, state_dict=None):
@@ -205,7 +208,7 @@ class HostReference:
             self.kind = "reference"
             self.model = self.ns2.Model(**CFG).eval()
             self.model.load_state_dict(sd)
-            self.desc = "unmodified reference Model.forward from baseline/_ref, torch fp32 CPU"
+            self.desc = "unmodified reference Model.forward from oracle/_ref, torch fp32 CPU"
         else:
             from oracle import denoiser_oracle, denoiser_torch_port
             self.kind = "port"
@@ -376,7 +379,7 @@ def secondary_aligner(dev, peaks):
                         "peak_GBps": float(peaks.get("hbm_gbs", 6650.0))}}
     try:
         if import_reference() is None:
-            raise RuntimeError("baseline/_ref is not present")
+            raise RuntimeError("oracle/_ref is not present")
         import time
         from naturalspeech2_pytorch.aligner import maximum_path as ref_mas
         torch.set_num_threads(_host_threads())
@@ -432,7 +435,7 @@ def secondary_prompt_encoder(dev, peaks):
     try:
         ns2 = import_reference()
         if ns2 is None:
-            raise RuntimeError("baseline/_ref is not present")
+            raise RuntimeError("oracle/_ref is not present")
         torch.set_num_threads(_host_threads())
         ref = ns2.SpeechPromptEncoder(dim_codebook=Dc).eval()
         ref.load_state_dict(enc.state_dict())
@@ -509,6 +512,21 @@ def train_step_dp(dev, world, peaks, steps=4, warmup=2):
     del opt, ns, model
     torch.cuda.empty_cache()
     return res
+
+
+def dump_outputs(out_dir, pred, loss_rows, loss):
+    """What one step of the timed path returns to its caller, as float32 `out_dir/<name>.npy`: `pred` = DUMP_ROWS
+    (sample, position) rows of the (32, 1024, 512) prediction, drawn with a fixed seed and kept in ascending flat row
+    order (DUMP_ROWS, 512); `loss_rows` = the per-sample MSE (32,); `loss` = the batch-mean loss ().  The inputs are
+    seeded too, so runs with the same arguments can be compared file by file across builds."""
+    import numpy as np
+    import torch
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    rows = torch.randperm(pred.shape[0] * pred.shape[1], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS]
+    rows = rows.sort().values.to(pred.device)
+    for name, t in (("pred", pred.reshape(-1, pred.shape[-1])[rows]), ("loss_rows", loss_rows), ("loss", loss)):
+        np.save(out_dir / f"{name}.npy", t.detach().float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -626,6 +644,8 @@ def run_ours(args):
     value = world * args.steps / (ms_total / 1e3)
     gpu_head = pred[:CPU_SAMPLE_BATCH].float().cpu()
     loss_value = float(losses[(args.steps - 1) & 1].item()) / world
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pred, loss_rows, losses[(args.steps - 1) & 1] / world)
 
     # ------------------------------- e2e: host buffers in, host buffers out --------------------------
     model.use_cuda_graphs = not args.no_cuda_graphs   # the public API call replays the model's own captured graph
@@ -818,7 +838,13 @@ def main():
     ap.add_argument("--no-cuda-graphs", action="store_true")
     ap.add_argument("--ref-max-batch", type=int, default=BATCH,
                     help="reference arm: cap on the per-step sample batch (tests use 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0) to DIR/<name>.npy, float32, 16 MiB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version banner at the first
     # collective, the reference prints a GPU notice at import): send file descriptor 1 to stderr for the whole run and
     # keep a private handle on the real stdout for the final line.

@@ -11,6 +11,8 @@ never sees /root/reference; it only reads the committed fixtures.
 """
 from __future__ import annotations
 
+import contextlib
+import inspect
 import sys
 import types
 from pathlib import Path
@@ -386,6 +388,59 @@ def aligner_goldens():
     print("aligner:", {k: v.shape for k, v in out.items() if k.endswith("_path")})
 
 
+# Drop-in surface (tests/test_dropin_cpu.py): BASELINE configs[0..2] (README model, cfg2, cfg3), a small conditional
+# model and the model the patch test rebinds.  Recorded per configuration: the reference Model's state_dict keys in
+# order with their shapes, and the attributes integration.infer_model_kwargs reads; plus the reference call signatures.
+DROPIN_CONFIGS = {
+    "cfg1_readme": dict(dim=128, depth=6),
+    "cfg2": dict(dim=512, depth=12, heads=8),
+    "cfg3": dict(dim=512, depth=12, dim_prompt=512, condition_on_prompt=True),
+    "small_cond": dict(dim=128, depth=2, heads=2, wavenet_layers=3, wavenet_stacks=2, dim_prompt=192,
+                       condition_on_prompt=True, resampler_depth=1, num_latents_m=16, cond_drop_prob=0.25),
+    "patch_small": dict(dim=128, depth=1, heads=2, wavenet_layers=2, wavenet_stacks=2),
+}
+DROPIN_SIGNATURES = ["Model.__init__", "Model.forward", "Model.forward_with_cond_scale", "NaturalSpeech2.forward",
+                     "NaturalSpeech2.sample"]
+
+
+@contextlib.contextmanager
+def shapes_only():
+    """Skip the (slow) random initialisation of nn.Linear / nn.Conv1d weights: parameters stay torch.empty."""
+    names = ("kaiming_uniform_", "uniform_", "normal_", "zeros_", "ones_", "trunc_normal_")
+    saved = {n: getattr(torch.nn.init, n) for n in names}
+    try:
+        for n in names:
+            setattr(torch.nn.init, n, lambda t, *a, **k: t)
+        yield
+    finally:
+        for n, f in saved.items():
+            setattr(torch.nn.init, n, f)
+
+
+def signature_spec(fn):
+    """(name, kind, repr(default)) of every parameter of `fn`."""
+    return [(p.name, p.kind.name, repr(p.default)) for p in inspect.signature(fn).parameters.values()]
+
+
+def dropin_goldens(ns2):
+    out = {}
+    for name, kwargs in DROPIN_CONFIGS.items():
+        with shapes_only():
+            m = ns2.Model(**kwargs)
+        attrs = dict(dim=m.dim, depth=len(m.transformer.layers), heads=m.transformer.layers[0][1].heads,
+                     wavenet_layers=len(m.wavenet.stacks[0].blocks), wavenet_stacks=len(m.wavenet.stacks),
+                     condition_on_prompt=bool(m.condition_on_prompt), cond_drop_prob=float(m.cond_drop_prob))
+        if m.condition_on_prompt:
+            attrs["resampler_depth"] = len(m.perceiver_resampler.layers)
+        out[f"{name}_keys"] = np.array(repr([(k, tuple(v.shape)) for k, v in m.state_dict().items()]))
+        out[f"{name}_attrs"] = np.array(repr(attrs))
+    for qual in DROPIN_SIGNATURES:
+        cls, meth = qual.split(".")
+        out[f"sig_{qual}"] = np.array(repr(signature_spec(getattr(getattr(ns2, cls), meth))))
+    np.savez_compressed(HERE / "dropin_surface.npz", **out)
+    print("dropin:", sorted(out))
+
+
 def math_log2(v):
     import math
     return math.log2(v)
@@ -410,6 +465,8 @@ def main():
         aligner_goldens()
     if not only or "encoders" in only:
         encoder_goldens(ns2)
+    if not only or "dropin" in only:
+        dropin_goldens(ns2)
 
 
 if __name__ == "__main__":

@@ -4,6 +4,8 @@ import subprocess
 import sys
 from pathlib import Path
 
+import pytest
+
 ROOT = Path(__file__).resolve().parent.parent
 
 
@@ -16,8 +18,9 @@ def test_reference_arm_json_contract():
     d = json.loads(line)
     assert d["impl"] == "reference" and d["metric"] == "denoiser-steps/sec" and d["unit"] == "steps/s"
     assert d["higher_is_better"] is True and d["value"] > 0
-    # baseline/_ref (the pip-installed reference) when present, else the oracle port
-    expect_kind = "reference" if (ROOT / "baseline" / "_ref" / "naturalspeech2_pytorch").exists() else "port"
+    # oracle/_ref (the pip-installed reference) when present, else the oracle port
+    from oracle import reference
+    expect_kind = "reference" if reference.installed() else "port"
     assert d["cpu_baseline"]["kind"] == expect_kind
     assert d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["steps"] == 2 and d["sample_batch"] == 2 and d["extrapolated"] is True
@@ -26,6 +29,14 @@ def test_reference_arm_json_contract():
     sys.path.insert(0, str(ROOT))
     import bench
     assert d["config"] == bench.build_config(1)   # both arms print the same config object
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_rejected_arguments(argv, tmp_path):
+    res = subprocess.run([sys.executable, str(ROOT / "bench.py"), *argv], capture_output=True, text=True, timeout=120,
+                         cwd=str(tmp_path))
+    assert res.returncode == 2 and res.stdout == "" and "error" in res.stderr
+    assert not (tmp_path / "out").exists()
 
 
 def test_reference_arm_other_ranks_exit_quietly():
